@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- views/sec forward+backward of the feature-Gaussian rasterizer (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c3] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -91,6 +91,58 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_BYTES = 60 << 20  # array data; with the .npy headers the files stay under 64 MB
+
+
+class OutputDump:
+    """--dump-outputs: what the timed `value` path computed in its last step, written as DIR/<name>.npy in float32.
+    Per-view outputs (color, feature_map, depth, radii and, through the autograd API, grad_means2D) are stacked over
+    this rank's views; the parameter gradients are the step's accumulated (all-reduced) ones.  So that the whole dump stays within DUMP_BYTES, an array with more than
+    `cap` elements is replaced by a fixed sample of its flat elements (sorted indices drawn with numpy PCG64 seed 0, the
+    same for every view and every run with the same arguments), stored as [views, cap] / [cap]."""
+
+    def __init__(self, n_views, n_arrays):
+        self.n_views, self.cap = n_views, DUMP_BYTES // 4 // n_arrays
+        self.sel, self.bufs = {}, {}
+
+    def _select(self, name, x):
+        import torch
+
+        if name not in self.sel:
+            n = x.numel()
+            self.sel[name] = None if n <= self.cap else torch.from_numpy(
+                np.sort(np.random.Generator(np.random.PCG64(0)).choice(n, self.cap, replace=False))).to(x.device)
+        return self.sel[name]
+
+    def keep(self, view, **outs):
+        """Inside the timed step: device-side copies / gathers into buffers allocated on the first (warm-up) step."""
+        import torch
+
+        for name, x in outs.items():
+            if x.numel() == 0:
+                continue
+            x = x.detach()
+            sel = self._select(name, x)
+            if name not in self.bufs:
+                shape = tuple(x.shape) if sel is None else (sel.numel(),)
+                self.bufs[name] = x.new_empty((self.n_views,) + shape)
+            if sel is None:
+                self.bufs[name][view].copy_(x)
+            else:
+                torch.index_select(x.reshape(-1), 0, sel, out=self.bufs[name][view])
+
+    def write(self, out_dir, grads):
+        arrays = dict(self.bufs)
+        for name, g in grads.items():
+            sel = self._select(name, g)
+            arrays[name] = g.detach() if sel is None else g.detach().reshape(-1)[sel]
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a.float().cpu().numpy())
+        log(f"dump-outputs: {len(arrays)} arrays to {out_dir}: " + ", ".join(
+            f"{k}{list(a.shape)}" for k, a in sorted(arrays.items())))
+
+
 def algorithmic_bytes(V, R, tiles, HW, C):
     """SURVEY.md section 8(d): compulsory traffic of the two composite kernels, bytes per view."""
     fwd = V * (4 * C + 40) + 4 * R + 8 * tiles + HW * (4 * C + 24)
@@ -155,7 +207,13 @@ def main():
                     help="write a 512 MB buffer between timed steps (outside the per-step event pairs)")
     ap.add_argument("--ref-debug", action="store_true",
                     help="reference arm only: debug=True, the reference scripts' default (arguments/__init__.py:71)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of `value`, write what its last step computed (per-view outputs and the "
+                         "step's gradients) to DIR/<name>.npy, float32, at most 64 MB (larger arrays as a fixed seeded "
+                         "sample); the copies run inside the timed steps")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     import torch
     import torch.distributed as dist
@@ -251,15 +309,18 @@ def main():
 
     def render(cam, packed):
         means2D = torch.zeros_like(t["means3D"], requires_grad=True)
+        if dump:
+            stats["means2D"] = means2D  # its .grad: the viewspace gradient a caller of the autograd API receives
         return make_rasterizer(cam, packed)(
             means3D=t["means3D"], means2D=means2D, opacities=t["opacities"], shs=t["shs"],
             semantic_feature=t["semantic_feature"] if C else None, scales=t["scales"], rotations=t["rotations"])
 
     # teacher feature map at the teacher's resolution (reference train.py:99: viewpoint_cam.semantic_feature), resident
     Hg, Wg = max(int(round(H / 2.25)), 1), max(int(round(W / 2.25)), 1)
-    gt_feat = torch.rand(C, Hg, Wg, device=dev) if C else None
+    gt_feat = torch.rand(C, Hg, Wg, device=dev, generator=torch.Generator(dev).manual_seed(7)) if C else None
 
     stats = {}
+    dump = OutputDump(len(cams), 5 * len(cams) + 8) if args.dump_outputs and rank == 0 else None
     use_batch = args.impl == "ours" and args.api == "batch" and not fwd_only
     if args.impl == "ours" and not fwd_only:
         vb = ViewBatch({k: t[k].detach() for k in ("means3D", "scales", "rotations", "opacities", "shs", "semantic_feature")})
@@ -274,6 +335,8 @@ def main():
             vb.zero_()
             for i, cam in enumerate(cams):
                 color, feat, radii, depth, ctx = vb.forward(settings_of(cam, cam_dev[i]))
+                if dump:
+                    dump.keep(i, color=color, feature_map=feat, depth=depth, radii=radii)
                 vb.backward(ctx, gc, gf if C else None, gd, last=(i == len(cams) - 1))
                 stats["radii"] = radii
             vb.all_reduce()
@@ -306,16 +369,22 @@ def main():
             with torch.no_grad():
                 for i, cam in enumerate(cams):
                     color, feat, radii, depth = render(cam, cam_dev[i])
+                    if dump:
+                        dump.keep(i, color=color, feature_map=feat, depth=depth, radii=radii)
                     stats["radii"] = radii
             return
         flat.zero_()
         for i, cam in enumerate(cams):
             color, feat, radii, depth = render(cam, cam_dev[i])
+            if dump:
+                dump.keep(i, color=color, feature_map=feat, depth=depth, radii=radii)
             outs, gos = [color, depth], [gc, gd]
             if C:
                 outs.append(feat)
                 gos.append(gf)
             torch.autograd.backward(outs, gos)
+            if dump:
+                dump.keep(i, grad_means2D=stats["means2D"].grad)
             stats["radii"] = radii
         flat.all_reduce()
 
@@ -401,6 +470,17 @@ def main():
         stage_ms, stage_cnt = _C.profile_read()
     views_per_step = n_views
     value = views_per_step * args.steps / (ms_total / 1000.0)
+    if dump:
+        if fwd_only:
+            grads = {}
+        elif use_batch:
+            grads = {"grad_" + k: g for k, g in vb.grads.items()}
+            grads.update(grad_accum=vb.grad_accum, denom=vb.denom)
+        else:
+            grads = {"grad_" + k: t[k].grad for k in ("means3D", "scales", "rotations", "opacities", "shs",
+                                                      "semantic_feature") if t[k].grad is not None}
+        dump.write(args.dump_outputs, grads)
+        dump = None  # the later regions run the same step functions
 
     # ---------------- timed region 2: end to end
     ms_e2e = timed(step_e2e_batch if use_batch else step_e2e, args.steps, max(args.warmup, 3))
@@ -445,6 +525,8 @@ def main():
                                 "(align_corners=True). Autograd API / reference arm: PyTorch operators; batch API: the fused "
                                 "feature head (csrc/feature_head.cu)")},
         "clocks": clocks,
+        "dump_outputs": (None if not args.dump_outputs else
+                         f"{args.dump_outputs}: the timed steps of `value` include the device-side copies of the dump"),
         "e2e": {"value": e2e_value, "unit": "views/s", "h2d_bytes_per_step": h2d_bytes, "d2h_bytes_per_step": 4,
                 "ms_per_step": ms_e2e / args.steps},
     }

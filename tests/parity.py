@@ -10,6 +10,7 @@ signed fp32 terms; the reference adds them with order-nondeterministic atomics (
 ~1e-6 of max|b|), we add them in a different (hierarchical) order.  Worst case over the test-suite so far:
 1.4e-5 of max|b| (grad_scales with a non-zero background), i.e. 7x inside the 1e-4 bound.
 """
+import hashlib
 import os
 import sys
 
@@ -205,6 +206,108 @@ def compare(ours, ref, int_keys=INT_KEYS, float_keys=FWD_FLOAT_KEYS, grad_keys=G
                 ok &= r <= 1.0
     rep["ok"] = bool(ok)
     return rep
+
+
+RECORD_EXACT_KEYS = ("color", "depth", "final_T")  # bit-identical to the reference build
+PIX_BLOCK = 64      # image moments: per 64 x 64-pixel block over all channels, and per channel over all pixels
+GAUSS_BLOCK = 4096  # gradient moments: per block of 4096 Gaussians over all components, and per component
+
+
+def _digest(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def _record_arrays(out):
+    """name -> (array in its canonical dtype, is_float, absolute-tolerance floor) of one run_ours()/run_oracle() result."""
+    arrs = {k: (np.asarray(out[k]).astype(np.int64), False, None) for k in INT_KEYS}
+    arrs.update({k: (np.asarray(out[k], np.float32), True, ATOL_REL) for k in FWD_FLOAT_KEYS})
+    for k, v in out.get("grads", {}).items():
+        if k in GRAD_KEYS:
+            arrs["grad_" + k] = (np.asarray(v, np.float32), True, GRAD_ATOL_REL)
+    return arrs
+
+
+def _moments(k, a):
+    """float64 (count, sum x, sum |x|, sum x^2) of `a` in two groupings that each cover every element: images ([C,H,W] or
+    [H,W]) per PIX_BLOCK x PIX_BLOCK pixels over all channels ("blk") and per channel over all pixels ("ch"); gradients
+    ([P, ...]) per GAUSS_BLOCK Gaussians over all components ("blk") and per component over all Gaussians ("ch").
+    -> {"blk": [4, blocks], "ch": [4, channels]}"""
+    def four(v):
+        return [np.ones_like(v), v, np.abs(v), v * v]
+
+    if k.startswith("grad_"):
+        x = a.reshape(a.shape[0], -1)
+        starts = range(0, x.shape[0], GAUSS_BLOCK)
+        blk, ch = np.zeros((4, len(starts))), np.zeros((4, x.shape[1]))
+        for i, r in enumerate(starts):
+            v = x[r:r + GAUSS_BLOCK].astype(np.float64)
+            sums = np.stack([m.sum(axis=0) for m in four(v)])
+            blk[:, i] = sums.sum(axis=1)
+            ch += sums
+        return {"blk": blk, "ch": ch}
+    x = a.reshape((-1,) + a.shape[-2:])
+    rows, cols = np.arange(0, x.shape[1], PIX_BLOCK), np.arange(0, x.shape[2], PIX_BLOCK)
+    blk, ch = np.zeros((4, len(rows), len(cols))), np.zeros((4, x.shape[0]))
+    for c in range(x.shape[0]):
+        for j, m in enumerate(four(x[c].astype(np.float64))):
+            blk[j] += np.add.reduceat(np.add.reduceat(m, rows, axis=0), cols, axis=1)
+            ch[j, c] = m.sum()
+    return {"blk": blk.reshape(4, -1), "ch": ch}
+
+
+def make_record(ours, orc):
+    """Compact stand-in for a full-size result.  From `ours` (this project's CUDA path, whose integer arrays and
+    RECORD_EXACT_KEYS were asserted bit-identical to the reference build): the shape and SHA-256 of every array (integer
+    arrays as int64, float arrays as float32).  From `orc` (the CPU oracle, the reference algorithm restated; see
+    run_oracle): for every float array, max |b| over the whole array and the _moments() sums (float32)."""
+    rec, bars = {}, _record_arrays(orc)
+    for k, (a, is_float, _) in _record_arrays(ours).items():
+        rec["shape_" + k] = np.asarray(a.shape, np.int64)
+        rec["sha256_" + k] = np.asarray(_digest(a))
+        if is_float and a.size:
+            b = bars[k][0]
+            assert b.shape == a.shape, (k, b.shape, a.shape)
+            rec["scale_" + k] = np.float64(np.max(np.abs(b)))
+            for g, m in _moments(k, b).items():
+                rec[f"{g}_{k}"] = m[1:].astype(np.float32)
+    return rec
+
+
+def check_record(ours, rec):
+    """Compare one run_ours() result with a make_record() record.  Integer arrays and RECORD_EXACT_KEYS must have the
+    recorded digest (bit-identical over the whole array).  Every float array must satisfy, in every block and channel of
+    _moments(), the bounds that the elementwise bar of compare(), |a-b| <= r|b| + q with r = RTOL and q = floor * max|b|,
+    implies for sums over the n elements of a block:
+        |sum a - sum b|, |sum |a| - sum |b||  <=  r sum|b| + n q
+        |sum a^2 - sum b^2|                   <=  (2r + r^2) sum b^2 + 2 (1 + r) q sum|b| + n q^2
+    (each widened by 2^-23 of its recorded magnitude for the float32 storage), so a result within the elementwise bar
+    always passes, while a wrong tile, channel or block of Gaussians shows up in its sums.
+    -> list of failure messages (empty: pass)."""
+    bad = []
+    arrs = _record_arrays(ours)
+    for k in (n[len("shape_"):] for n in rec.files if n.startswith("shape_")):
+        if k not in arrs:
+            bad.append(f"{k}: missing from the result")
+            continue
+        a, is_float, atol_rel = arrs[k]
+        want_shape = tuple(int(s) for s in rec["shape_" + k])
+        if a.shape != want_shape:
+            bad.append(f"{k}: shape {a.shape} != recorded {want_shape}")
+            continue
+        if (not is_float or k in RECORD_EXACT_KEYS) and _digest(a) != str(rec["sha256_" + k]):
+            bad.append(f"{k}: not bit-identical to the record")
+        if not (is_float and ("blk_" + k) in rec.files):
+            continue
+        r, q, eps = RTOL, atol_rel * float(rec["scale_" + k]), 2.0 ** -23
+        for g, (n, s1, sa, s2) in _moments(k, a).items():
+            b1, ba, b2 = rec[f"{g}_{k}"].astype(np.float64)
+            t1 = r * ba + n * q + eps * ba + 1e-30
+            t2 = (2 * r + r * r) * b2 + 2 * (1 + r) * q * ba + n * q * q + eps * b2 + 1e-30
+            viol = np.max(np.stack([np.abs(s1 - b1) / t1, np.abs(sa - ba) / t1, np.abs(s2 - b2) / t2]), axis=0)
+            worst = int(np.argmax(np.where(np.isfinite(viol), viol, np.inf)))
+            if not np.all(np.isfinite(viol)) or viol[worst] > 1.0:
+                bad.append(f"{k}: {g} sums outside the bar, worst {float(viol[worst]):.3g} at {g} {worst} of {viol.size}")
+    return bad
 
 
 def format_report(rep):

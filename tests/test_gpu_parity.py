@@ -1,7 +1,8 @@
 """GPU parity tests proper (-m gpu): this repo's CUDA path, called through the public Python API -> torch
 binding -> C ABI, against
-  * the UNMODIFIED reference CUDA extension (oracle/_ref, where a build for that feature width travels), and
-  * the CPU oracle (oracle/) for every case small enough,
+  * the UNMODIFIED reference CUDA extension (oracle/_ref, where a build for that feature width is present),
+  * the CPU oracle (oracle/) for every case small enough, and
+  * stored records (tests/golden/records, tests/make_records.py) for the full-size configs 2-5,
 on identical seeded inputs.  Bars (BASELINE.json north_star): bit-exact tile/key indexing (radii,
 num_rendered, point_list, ranges, n_contrib); RGB/feature/depth/gradients within 1e-4 relative
 (parity.RTOL + ATOL_REL floor).  On top of the bar, colour / depth / final_T are asserted BIT-identical to
@@ -9,6 +10,7 @@ the reference build (same fp32 operation sequence), the feature map to 5e-6 of i
 Nothing here reads /root/reference.
 """
 import copy
+import os
 
 import numpy as np
 import pytest
@@ -25,10 +27,21 @@ def _ref_available(C):
     return rw.available(C)
 
 
-def _check(sc, cam, with_grads=True, vs_ref=True, vs_oracle=True, exact_vs_ref=True, **kw):
+def _check_record(ours, name):
+    """Against the stored record of a full-size case (tests/make_records.py, parity.check_record): bit-exact digests of
+    the indices and of colour / depth / final_T, and the CPU oracle's block and channel sums for every float array."""
+    rec = np.load(os.path.join(os.path.dirname(__file__), "golden", "records", name + ".npz"))
+    bad = parity.check_record(ours, rec)
+    assert not bad, f"vs stored record {name} ({rec['gpu']}):\n  " + "\n  ".join(bad)
+
+
+def _check(sc, cam, with_grads=True, vs_ref=True, vs_oracle=True, exact_vs_ref=True, record=None, **kw):
     grads = scenegen.upstream_grads(cam.image_height, cam.image_width, sc.C) if with_grads else None
     ours = parity.run_ours(sc, cam, grads=grads, **kw)
     n = 0
+    if record is not None:
+        _check_record(ours, record)
+        n += 1
     if vs_ref and _ref_available(sc.C) and not kw:
         ref = parity.run_ref(sc, cam, grads=grads)
         rep = parity.compare(ours, ref)
@@ -62,7 +75,7 @@ def test_small_configs_vs_reference_and_oracle(name):
 
 def test_c2_vs_reference():
     sc = scenegen.make_config("c2")
-    _check(sc, sc.cameras[0], vs_oracle=False)
+    _check(sc, sc.cameras[0], vs_oracle=False, record="c2")
 
 
 def test_golden_fixtures_match_gpu():
@@ -300,16 +313,18 @@ def c3_scene():
 
 
 def _full_size_vs_reference(sc, with_grads, label):
-    """Device-side comparison of one full-size view against the reference build; prints the worst violation ratio
-    (|a-b| / tolerance, <= 1 passes) of every float tensor so the margin is on record in the test log."""
+    """One full-size view against its stored record and, where a reference build for this width is present, device-side
+    against the reference build; the latter prints the worst violation ratio (|a-b| / tolerance, <= 1 passes) of every
+    float tensor so the margin is on record in the test log."""
     import torch
     from oracle import ref_wrapper as rw
 
-    if not rw.available(sc.C):
-        pytest.skip(f"no reference build for C={sc.C} on this box")
     cam = sc.cameras[0]
     grads = scenegen.upstream_grads(cam.image_height, cam.image_width, sc.C) if with_grads else None
     ours = parity.run_ours(sc, cam, grads=grads)
+    _check_record(ours, label)
+    if not rw.available(sc.C):
+        return
     ref = parity.run_ref(sc, cam, grads=grads)
     for k in ("radii", "point_list", "ranges", "n_contrib"):
         assert np.array_equal(ours[k], ref[k]), k
